@@ -25,7 +25,7 @@ from patchfusion_b200.params import synthetic_state_dict             # noqa: E40
 
 GOLD = os.path.join(ROOT, 'tests', 'golden')
 CASE = dict(encoder='vits', seed=0, image_raw_shape=(1080, 1920), patch_split_num=(2, 2), process_num=2,
-            input_seed=0, sample_stride=4)
+            input_seed=0, sample_stride=8)        # stride 8 keeps tests/golden/vits_case0.npz under 1 MB
 
 
 def sample(t, stride):
